@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus 1 --steps 20 --warmup 5   # the reference's CPU path (oracle port)
     torchrun ... bench.py --gpus N ...                                # one replica of the workload per rank
     python bench.py --workload small_upsampler | 5b_lyrics | vqvae_decode   # BASELINE configs[2], [3], [4]
+    python bench.py ... --dump-outputs DIR                            # + what the last timed step computed, DIR/*.npy
 
 Default workload "1b_lyrics": SimplePrior (prior_1b_lyrics hparams, n_ctx=8192 override -> 8576 positions incl.
 384 lyric tokens), n_samples=16 per GPU, random-init synthetic weights, random labels and lyric tokens, fp16
@@ -69,7 +70,11 @@ def parse():
     ap.add_argument("--small", action="store_true", help="tiny debug configuration (not a valid bench number)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (rank 0), to compare two builds")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm has none")
     if a.workload == "prior":
         a.workload = "1b_lyrics"
     return a
@@ -265,6 +270,35 @@ def load_peaks():
         return {}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE = 1 << 20          # elements kept of an output too large to dump whole
+
+
+def dump_outputs(out_dir, arrays):
+    """name -> float32 / float64 array, written as out_dir/<name>.npy (at most DUMP_LIMIT_BYTES in all)"""
+    import numpy as np
+    arrays = {k: np.ascontiguousarray(v) for k, v in arrays.items()}
+    assert all(v.dtype in (np.float32, np.float64) for v in arrays.values())
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"{total} bytes of outputs exceed the dump limit of {DUMP_LIMIT_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
+def sample_of(x):
+    """a fixed sample of DUMP_SAMPLE elements of a large CUDA tensor, flattened (indices seeded, sorted): the same
+    positions from run to run for the same shape"""
+    import numpy as np
+    import torch
+    flat = x.reshape(-1)
+    if flat.numel() <= DUMP_SAMPLE:
+        return flat.cpu().numpy()
+    idx = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_SAMPLE, replace=False))
+    return flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy()
+
+
 # ----------------------------------------------------------------------------------------------
 # CPU arm: the oracle (numpy restatement of the reference's CA2D.sample body) on the host cores
 # ----------------------------------------------------------------------------------------------
@@ -410,10 +444,11 @@ def run_reference(args, rank, world):
 
 
 # ----------------------------------------------------------------------------------------------
-def measure_vqvae(args, rank, world, local, steps, warmup, small=False):
+def measure_vqvae(args, rank, world, local, steps, warmup, small=False, dump=None):
     """BASELINE configs[4]: 3-level VQ-VAE decode, sample_length 1048576, bs 16 per GPU; one step = every
     clip decoded at every level exactly as sample.py:108 does (decode(zs[l:], start_level=l, bs_chunks=N)).
-    Returns the result dict (all ranks; times are max over ranks)."""
+    Returns the result dict (all ranks; times are max over ranks).  `dump`: directory that receives the audio the
+    last timed step decoded from each start level l, a fixed sample of it (sample_of), as audio_level<l>.npy."""
     import torch
     import torch.distributed as dist
     from jukebox_b200.hparams import setup_hparams
@@ -441,12 +476,17 @@ def measure_vqvae(args, rank, world, local, steps, warmup, small=False):
         dist.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     c0 = _lib.CALLS
+    last = None
     e0.record()
     for _ in range(steps):
-        step(zs_dev)
+        last = None                    # one step's audio is freed before the next is decoded, as when discarded
+        last = step(zs_dev)
     e1.record()
     torch.cuda.synchronize()
     launches = _lib.CALLS - c0
+    if dump and rank == 0:
+        dump_outputs(dump, {f"audio_level{l}": sample_of(x) for l, x in enumerate(last)})
+    del last
     ms = torch.tensor([e0.elapsed_time(e1)], device="cuda")
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -509,7 +549,7 @@ def main():
         from jukebox_b200.utils.dist_sampling import scatter_rows, gather_rows, seed_per_rank
     seed_per_rank(0)
     if args.workload == "vqvae_decode":
-        res = measure_vqvae(args, rank, world, local, args.steps, args.warmup, args.small)
+        res = measure_vqvae(args, rank, world, local, args.steps, args.warmup, args.small, dump=args.dump_outputs)
         if rank == 0:
             res["vs_baseline"] = None
             print(json.dumps(res))
@@ -572,7 +612,9 @@ def main():
         if k == 0:
             state["win"] = begin_window()
         win = state["win"]
+        lo = win.pos
         win.advance(win.P + per_slice * (k + 1) if k < N_SLICES - 1 else win.sample_tokens)
+        state["last"] = (win, lo, win.pos)         # positions this step sampled (--dump-outputs)
         if k == N_SLICES - 1:
             if prior.single_enc_dec:
                 prior.prior_postprocess(win.finish())
@@ -603,6 +645,12 @@ def main():
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_value = float(ms)
+    if args.dump_outputs and rank == 0:
+        # the codes the last timed step sampled (token ids of the window, exact in float64) and the logits of its last
+        # position; same arguments, same inputs: weights, labels and the sampler's Philox key all come from fixed seeds
+        win, lo, hi = state["last"]
+        dump_outputs(args.dump_outputs, dict(tokens=win.tokens[:, lo:hi].double().cpu().numpy(),
+                                             logits=win.lbuf.float().cpu().numpy()))
     with quiet:                                # run the open window to its end (engine back to a clean state)
         while state["k"] != 0:
             slice_step()

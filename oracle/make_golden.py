@@ -3,6 +3,7 @@
 Run in the build container only (needs /root/reference):
 
     python -m oracle.make_golden            # rewrites every fixture
+    python -m oracle.make_golden hparams sample_level     # only the named golden_* fixtures
 
 Each fixture stores: a JSON config, the (name, shape) list of the reference module's
 state_dict, the seed the synthetic weights were drawn with (oracle/synth.py), the inputs
@@ -236,16 +237,37 @@ def golden_hparams():
     out = dict(registry={k: clean(v) for k, v in HPARAMS_REGISTRY.items()},
                defaults={k: clean(v) for k, v in DEFAULTS.items()},
                models={k: list(v) for k, v in MODELS.items()},
-               resolved={k: clean(setup_hparams(k, {})) for k in HPARAMS_REGISTRY})
+               resolved={k: clean(setup_hparams(k, {})) for k in HPARAMS_REGISTRY},
+               # Python literals keep what JSON loses: which values are tuples (ast.literal_eval reads them back)
+               resolved_repr={k: repr(dict(setup_hparams(k, {}))) for k in HPARAMS_REGISTRY})
     path = os.path.join(GOLDEN, "hparams.json")
     with open(path, "w") as f:
         json.dump(out, f, indent=0, sort_keys=True)
     print("wrote", path)
 
 
+def golden_sample_level():
+    """the reference's window planning / stitching (jukebox/sample.py:17-96) driven by the recording dummy prior of
+    tests/test_sample_plan_cpu.py, one record per case"""
+    import jukebox.sample as ref
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from test_sample_plan_cpu import CASES, case_id, run_sample_level
+    out = {}
+    for case in CASES:
+        total, n_ctx, hop, have, bs, mbs = case
+        if total >= n_ctx and have > total:
+            continue
+        out[case_id(case)] = run_sample_level(ref, *case)
+    path = os.path.join(GOLDEN, "sample_level.json")
+    with open(path, "w") as f:
+        json.dump(out, f, sort_keys=True)
+    print("wrote", path)
+
+
 def main():
     os.makedirs(GOLDEN, exist_ok=True)
     golden_hparams()
+    golden_sample_level()
     golden_transformer("order9", n_in=64, n_ctx=48, n_head=2, n_depth=8, attn_order=9, blocks=4, bs=3)
     golden_transformer("order6", n_in=64, n_ctx=48, n_head=2, n_depth=8, attn_order=6, blocks=4, bs=2,
                        encoder_dims=10)
@@ -262,4 +284,9 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) > 1:
+        os.makedirs(GOLDEN, exist_ok=True)
+        for name in sys.argv[1:]:
+            globals()["golden_" + name]()
+    else:
+        main()

@@ -1,12 +1,15 @@
 """Window planning / stitching of jukebox_b200.sample against the UNMODIFIED reference's own loop
-(jukebox/sample.py:17-96), both driven with the same recording dummy prior on the CPU.  Skipped when the reference
-tree is absent (GPU box)."""
+(jukebox/sample.py:17-96), both driven with the same recording dummy prior on the CPU.  What the reference's loop
+returned and how it called the prior, case by case, is pinned in tests/golden/sample_level.json
+(oracle/make_golden.py: golden_sample_level)."""
 import itertools
+import json
+import os
 
 import pytest
 import torch
 
-from oracle.ref_import import reference_available, load_reference
+from golden_util import GOLDEN
 from jukebox_b200.sample import plan_windows, Window
 from jukebox_b200.utils.sample_utils import get_starts
 
@@ -42,31 +45,37 @@ CASES = [(total, n_ctx, hop, have, bs, mbs)
          for have in (0, 3, 11, 16, 20) for bs, mbs in ((3, 2), (4, 4))]
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not present")
+def case_id(case):
+    return "-".join(str(v) for v in case)
+
+
+def run_sample_level(mod, total, n_ctx, hop, have, bs, mbs):
+    """`mod.sample_level` on one case: {"zs": codes, "calls": prior calls} as JSON values, or {"error": type name}"""
+    prior = RecordingPrior(n_ctx)
+    zs = [torch.arange(have).view(1, -1).repeat(bs, 1)]
+    hps = Hps(n_samples=bs)
+    kw = dict(temp=0.9, fp16=True, max_batch_size=mbs)
+    try:
+        zs = mod.sample_level(zs, None, kw, 0, prior, total, hop, hps)
+    except Exception as e:              # both sides must fail alike (e.g. negative slices)
+        return dict(error=type(e).__name__)
+    return dict(zs=zs[0].tolist(), calls=[[n, p, t, list(keys)] for n, p, t, keys in prior.calls])
+
+
 @pytest.mark.parametrize("total,n_ctx,hop,have,bs,mbs", CASES)
 def test_sample_level_matches_reference(total, n_ctx, hop, have, bs, mbs):
-    load_reference()
-    import jukebox.sample as ref
     import jukebox_b200.sample as ours
     if total >= n_ctx and have > total:
         pytest.skip("more tokens than the level holds")
-    outs = []
-    for mod in (ref, ours):
-        prior = RecordingPrior(n_ctx)
-        zs = [torch.arange(have).view(1, -1).repeat(bs, 1)]
-        hps = Hps(n_samples=bs)
-        kw = dict(temp=0.9, fp16=True, max_batch_size=mbs)
-        try:
-            zs = mod.sample_level(zs, None, kw, 0, prior, total, hop, hps)
-            outs.append((zs[0].clone(), prior.calls))
-        except Exception as e:          # both sides must fail alike (e.g. negative slices)
-            outs.append(("error", type(e).__name__))
-    if outs[0][0] == "error" if isinstance(outs[0][0], str) else False:
-        assert isinstance(outs[1][0], str)
+    with open(os.path.join(GOLDEN, "sample_level.json")) as f:
+        want = json.load(f)[case_id((total, n_ctx, hop, have, bs, mbs))]
+    got = run_sample_level(ours, total, n_ctx, hop, have, bs, mbs)
+    if "error" in want:
+        assert "error" in got, got
         return
-    assert not isinstance(outs[1][0], str), outs[1]
-    assert torch.equal(outs[0][0], outs[1][0])
-    assert outs[0][1] == outs[1][1]
+    assert "error" not in got, got
+    assert got["zs"] == want["zs"]
+    assert got["calls"] == want["calls"]
 
 
 def test_plan_windows_shapes():

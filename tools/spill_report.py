@@ -1,6 +1,6 @@
 """Per-device-function register / spill report of the decode kernel (CPU only, ~1 min).
 
-    python tools/spill_report.py            # compiles jukebox_b200/csrc/decode_engine.cu to /tmp and analyses it
+    python tools/spill_report.py            # compiles jukebox_b200/csrc/decode_engine.cu to a temporary directory and analyses it
     python tools/spill_report.py file.o     # analyse an existing object
 
 Why it exists: the persistent kernel runs 9 warps per CTA, which caps it at 168 registers, and ptxas'
@@ -10,12 +10,13 @@ part of its load batch; the STL then waits for the load and serialises everythin
 GEMM phase, +400 us per token).  stage_acts must report STL 0 / LDL 0 before a kernel change is measured.
 """
 import os
-import re,sys,subprocess
+import re,sys,subprocess,tempfile
 if len(sys.argv) > 1:
     o = sys.argv[1]
 else:
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    o = "/tmp/jk_decode_engine_spill.o"
+    tmp = tempfile.TemporaryDirectory()     # private per run: a fixed shared path may belong to another user
+    o = os.path.join(tmp.name, "jk_decode_engine_spill.o")
     subprocess.run(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "--expt-relaxed-constexpr",
                     "-c", os.path.join(root, "jukebox_b200", "csrc", "decode_engine.cu"), "-o", o], check=True)
 sass=subprocess.run(f"cuobjdump -sass {o}", shell=True, capture_output=True, text=True).stdout.splitlines()
